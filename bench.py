@@ -2,6 +2,7 @@
 """bench.py — benchmark of the hot path (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cuda|reference] [--workload NAME] [--replicas R] [--lpr L]
+                    [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs; default fifo60k = the configuration the metric "simulated events/sec on 60k-job trace" is
 quoted on and the only one with a measured reference number on that trace):
@@ -261,6 +262,47 @@ def load_profile(name):
         return None
 
 
+def dump_outputs(out_dir, sim, env, R, rows, returns):
+    """What the timed path returned in its last step, as float64 .npy files (at most 64 MB): `returns`, the episode return of
+    every replica of every GPU (rank-major, as all-gathered); every summary field of this GPU's replicas; the job tables and, with
+    rows, the per-tick / per-event rows of a seeded sample of this GPU's replicas (rows themselves a seeded sample above 65 536
+    per replica; `rows_index` names them).  The arrays of the sampled replicas are concatenated in replica order; `<table>_len`
+    holds each replica's length.  Rank 0 writes them."""
+    import numpy as np
+    from rlgpuschedule_b200 import _ffi
+    rng = np.random.default_rng(0)
+    out = {}
+
+    def put(name, arrs):
+        out[name] = np.concatenate([np.asarray(x, np.float64) for x in arrs])
+        out[name + '_len'] = np.array([len(x) for x in arrs], np.float64)
+
+    summ = [sim.summary(r) for r in range(R)]
+    out.update({'summary_' + f: np.array([s[f] for s in summ], np.float64) for f, _ in _ffi.Summary._fields_})
+    out['returns'] = np.asarray(returns, np.float64)
+    if env is not None:
+        out.update(env_obs=env.obs.double().cpu().numpy(), env_reward=env.reward.double().cpu().numpy(),
+                   env_done=env.done.double().cpu().numpy())
+    pick = np.sort(rng.choice(R, min(R, 4), replace=False))
+    out['sample_replicas'] = pick.astype(np.float64)
+    jobs = [sim.jobs(int(r)) for r in pick]
+    for k in ('start', 'end', 'finish_order', 'preempt'):
+        put('jobs_' + k, [j[k] for j in jobs])
+    if rows:
+        rs = [sim.rows(int(r)) for r in pick]
+        idx = [np.sort(rng.choice(len(x), 65536, replace=False)) if len(x) > 65536 else np.arange(len(x)) for x in rs]
+        put('rows_index', idx)
+        for f in _ffi.ROW_DTYPE.names:
+            out['rows_' + f] = np.concatenate([x[f][i].astype(np.float64) for x, i in zip(rs, idx)])
+    bad = [name for name, a in out.items() if not np.isfinite(a).all()]
+    assert not bad, 'outputs that are not finite: %s' % bad
+    total = sum(a.nbytes for a in out.values())
+    assert total <= 64 << 20, 'outputs to dump: %d bytes' % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -274,7 +316,10 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-python-reference', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy (float64)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'cuda':
+        ap.error('--dump-outputs writes what the timed cuda path computed: it needs --impl cuda')
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -401,6 +446,8 @@ def main():
     value = events_all * args.steps / dt_max
     jmax = max(len(tr.records) for tr in traces)
     max_ticks = max(s['n_ticks'] for s in summ)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sim, env, R, rows=not is_env, returns=gathered.cpu().numpy() if world > 1 else sim.returns())
     (env or sim).close()
 
     # ---------------- end-to-end arm through the C ABI with host buffers

@@ -255,3 +255,47 @@ CASES.update({
     'dlas_multi_node': dict(frame=_multi_node, flags=dict(num_switch=2, num_node_p_switch=2, num_gpu_p_node=4), schedule='dlas', queue_limit=(8, 12)),
     'dlas_probe2k': dict(frame=lambda: tg.frame_gen(2000, 1, 2000), flags=C4328, schedule='dlas', queue_limit=(30, 60, 150), big=True),
 })
+
+
+# ---- random traces and cluster shapes, recorded from the reference by `python oracle/make_golden.py --random` into
+# tests/golden/random_cases.json.gz (tests/test_oracle_vs_live_reference.py; tests/test_gpu_random.py draws from the same generator)
+RANDOM_GOLD = 'random_cases.json.gz'
+RANDOM_PACK_COMBOS = [('horus', 'horus'), ('gandiva', 'gandiva'), ('horus+', 'horus+'), ('horus', 'yarn'), ('gandiva', 'yarn'), ('horus+', 'yarn')]
+RANDOM_FIFO = list(range(100, 112))
+RANDOM_PACK = [(200 + 3 * i + j, combo) for i, combo in enumerate(RANDOM_PACK_COMBOS) for j in range(2)]
+RANDOM_LEGACY = [(300 + 5 * i + j, sched) for i, sched in enumerate(LEGACY) for j in range(2)]
+
+
+def random_case(seed):
+    rng = np.random.default_rng(seed)
+    n = int(rng.integers(20, 90))
+    flags = dict(num_switch=int(rng.integers(1, 3)), num_node_p_switch=int(rng.integers(1, 5)),
+                 num_gpu_p_node=int(rng.choice([2, 4, 8])), num_cpu_p_node=int(rng.choice([24, 48, 128])),
+                 mem_p_node=int(rng.choice([120, 256, 512])), gpu_memory_capacity=int(rng.choice([8, 16, 32])))
+    g = rng.choice([1, 2, 3, 4, 6, 8, 16], n)
+    gpc = np.array([int(rng.choice([c for c in (1, 2, 3, 4, 8) if c <= x])) for x in g])
+    rows = [dict(normalized_time=float(t), minutes=float(m), used_gpus=float(a), gpu_per_container=int(b),
+                 memory_max=int(mm), gpu_utilization_avg=float(u), gpu_utilization_max=float(min(100, u + 10)))
+            for t, m, a, b, mm, u in zip(np.sort(rng.uniform(0, 6e5, n)).round(-3 if seed % 2 else 0), rng.uniform(0.5, 60, n), g, gpc,
+                                         rng.uniform(5e8, 1.9e10, n), rng.uniform(1, 90, n))]
+    return tg.frame_rows(rows), flags
+
+
+def random_pack_case(seed, sched, scheme):
+    """Trace, flags and (look-ahead, queue count, k-means injection seed) of a random pack-family case; over the pack placement
+    the trace has zero utilisation spread (the reference's draws return their mean)."""
+    df, flags = random_case(seed)
+    if scheme != 'yarn':
+        df = df.copy(); df['gpu_utilization_max'] = df['gpu_utilization_avg']
+    rng = np.random.default_rng(seed + 7)
+    k = int(rng.integers(1, 8)); kq = int(rng.integers(1, 5)); inj = int(rng.integers(1, 1000))
+    return df, flags, k, kq, inj
+
+
+def random_legacy_queue_limit(seed):
+    rng = np.random.default_rng(seed + 11)
+    return tuple(int(x) for x in np.cumsum(rng.integers(5, 60, int(rng.integers(1, 4)))))   # 2 .. 4 queues
+
+
+def random_key(family, seed, *rest):
+    return '/'.join((family, str(seed)) + rest)

@@ -1,6 +1,7 @@
 """Generate tests/golden/* by running the real reference (oracle/ref_runner.py) in this container.
 
     python oracle/make_golden.py [case ...]        # default: every case not yet generated
+    python oracle/make_golden.py --random          # the random cases of golden_cases.RANDOM_* -> tests/golden/random_cases.json.gz
 
 Per case it stores: trace.csv (small cases; big ones are regenerated from tracegen seeds and
 checked by sha256), job.csv and cluster_noutil.csv exactly as the reference wrote them (CRLF
@@ -101,7 +102,49 @@ def make_legacy(name, case, out, work, trace, flags, big):
     return name, meta['n_events'], meta['n_job_rows'], meta['reference_wall_s']
 
 
+def _random_one(arg):
+    """One random case through the reference: its files, the sha256 of the trace it read, and how it ended."""
+    family, seed, rest = arg
+    work = tempfile.mkdtemp(prefix='rlgs_gold_random_%d_' % seed)
+    trace = os.path.join(work, 't.csv')
+    if family == 'legacy':
+        import ref_legacy_runner
+        df, flags = golden_cases.random_case(seed)
+        tracegen.write(df, trace)
+        ql = golden_cases.random_legacy_queue_limit(seed)
+        res = ref_legacy_runner.run_legacy(trace, rest[0], workdir=work, queue_limit=ql, **flags)
+        clu = res['cluster_csv']
+    else:
+        if family == 'fifo':
+            df, flags = golden_cases.random_case(seed)
+            extra = {}
+        else:
+            sched, scheme = rest
+            df, flags, k, kq, inj = golden_cases.random_pack_case(seed, sched, scheme)
+            extra = dict(schedule=sched, scheme=scheme, num_buffer=k, **(dict(num_queue=kq, inject_seed=inj) if sched == 'horus+' else {}))
+        tracegen.write(df, trace)
+        res = ref_runner.run_reference(trace, workdir=work, **extra, **flags)
+        clu = ref_runner.strip_util_column(res['cluster_csv']) if res['cluster_csv'] is not None else None
+    rec = dict(trace_sha256=sha(open(trace, 'rb').read()), job_csv=res['job_csv'], cluster_csv=clu,
+               returncode=res.get('returncode'), stderr_has_error='Error' in res['stderr'])
+    return golden_cases.random_key(family, seed, *rest), rec
+
+
+def make_random():
+    args = ([('fifo', s, ()) for s in golden_cases.RANDOM_FIFO] + [('pack', s, combo) for s, combo in golden_cases.RANDOM_PACK]
+            + [('legacy', s, (sched,)) for s, sched in golden_cases.RANDOM_LEGACY])
+    with ProcessPoolExecutor(max_workers=int(os.environ.get('GOLD_JOBS', '6'))) as ex:
+        out = dict(ex.map(_random_one, args))
+    fn = os.path.join(GOLD, golden_cases.RANDOM_GOLD)
+    with gzip.GzipFile(fn, 'wb', mtime=0) as f:
+        f.write(json.dumps(out, indent=0, sort_keys=True).encode())
+    return fn, len(out)
+
+
 if __name__ == '__main__':
+    if sys.argv[1:] == ['--random']:
+        print(*make_random())
+        sys.exit(0)
     names = sys.argv[1:] or [n for n in golden_cases.CASES
                              if not os.path.exists(os.path.join(GOLD, n, 'meta.json'))]
     with ProcessPoolExecutor(max_workers=int(os.environ.get('GOLD_JOBS', '6'))) as ex:

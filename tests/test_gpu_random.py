@@ -1,12 +1,12 @@
 """Randomised differential tests on the device: 60 random traces x cluster shapes, every schedule, against the
-CPU oracle (which tests/test_oracle_vs_live_reference.py ties to the live reference on the same generator)."""
+CPU oracle (which tests/test_oracle_vs_live_reference.py ties to the reference's recorded files on the same generator)."""
 import numpy as np
 import pytest
 
 import cpu_sim
+from golden_cases import random_case
 import rlgpuschedule_b200 as rl
 from rlgpuschedule_b200 import _ffi, log_manager as lm, synth
-from test_oracle_vs_live_reference import _case
 
 pytestmark = pytest.mark.gpu
 
@@ -14,7 +14,7 @@ pytestmark = pytest.mark.gpu
 @pytest.mark.parametrize('block', range(6))
 def test_random_cases_all_schedules(block):
     for seed in range(200 + 10 * block, 210 + 10 * block):
-        df, flags = _case(seed)
+        df, flags = random_case(seed)
         cluster = rl.cluster_from_flags(flags)
         tr = rl.prepare_trace(df, cluster)
         otr = cpu_sim.prepare_trace(df)
@@ -50,10 +50,10 @@ PACK_COMBOS = [('horus', 'horus'), ('gandiva', 'gandiva'), ('horus+', 'horus+'),
 
 @pytest.mark.parametrize('sched,scheme', PACK_COMBOS)
 def test_random_cases_pack_family(sched, scheme):
-    """The same generator as the live differential test of the oracle (tests/test_oracle_vs_live_reference.py): device vs oracle
+    """The same generator as the oracle's differential test against the reference (tests/test_oracle_vs_live_reference.py): device vs oracle
     on random traces / cluster shapes / look-ahead / queue counts, mean and seeded utilisation draws."""
     for seed in range(300, 312):
-        df, flags = _case(seed)
+        df, flags = random_case(seed)
         rng = np.random.default_rng(seed + 7)
         k = int(rng.integers(1, 8)); kq = int(rng.integers(1, 5)); inj = int(rng.integers(1, 1000))
         draws = bool(seed % 3 == 0) and scheme != 'yarn'        # every third case: seeded utilisation draws on the real spread

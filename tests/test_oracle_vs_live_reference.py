@@ -1,116 +1,71 @@
-"""Randomised differential test: oracle/cpu_sim.c vs the UNMODIFIED reference run live (only where
-/root/reference is mounted, i.e. in the build container; skipped on the GPU box).  Complements the fixed
-golden cases with fresh random traces / cluster shapes on every seed listed here."""
+"""Randomised differential test: oracle/cpu_sim.c vs the UNMODIFIED reference on random traces / cluster shapes.
+The reference's files for every seed listed in oracle/golden_cases.py (RANDOM_*) were recorded from live runs by
+`python oracle/make_golden.py --random` into tests/golden/random_cases.json.gz; the oracle is run here and compared with
+them byte for byte.  Complements the fixed golden cases."""
+import gzip
+import io
+import json
 import os
-import tempfile
-from concurrent.futures import ThreadPoolExecutor
 
-import numpy as np
+import pandas as pd
 import pytest
 
 import cpu_sim
-import ref_runner
-from rlgpuschedule_b200 import synth
-
-pytestmark = pytest.mark.skipif(not ref_runner.available(), reason='reference not mounted')
+import golden_cases
+import goldutil
 
 
-def _case(seed):
-    rng = np.random.default_rng(seed)
-    n = int(rng.integers(20, 90))
-    flags = dict(num_switch=int(rng.integers(1, 3)), num_node_p_switch=int(rng.integers(1, 5)),
-                 num_gpu_p_node=int(rng.choice([2, 4, 8])), num_cpu_p_node=int(rng.choice([24, 48, 128])),
-                 mem_p_node=int(rng.choice([120, 256, 512])), gpu_memory_capacity=int(rng.choice([8, 16, 32])))
-    g = rng.choice([1, 2, 3, 4, 6, 8, 16], n)
-    gpc = np.array([int(rng.choice([c for c in (1, 2, 3, 4, 8) if c <= x])) for x in g])
-    rows = [dict(normalized_time=float(t), minutes=float(m), used_gpus=float(a), gpu_per_container=int(b),
-                 memory_max=int(mm), gpu_utilization_avg=float(u), gpu_utilization_max=float(min(100, u + 10)))
-            for t, m, a, b, mm, u in zip(np.sort(rng.uniform(0, 6e5, n)).round(-3 if seed % 2 else 0), rng.uniform(0.5, 60, n), g, gpc,
-                                         rng.uniform(5e8, 1.9e10, n), rng.uniform(1, 90, n))]
-    return synth.frame_rows(rows), flags
+@pytest.fixture(scope='module')
+def recorded():
+    with gzip.open(os.path.join(goldutil.GOLD, golden_cases.RANDOM_GOLD), 'rt') as f:
+        return json.load(f)
 
 
-def _run(seed):
-    df, flags = _case(seed)
-    work = tempfile.mkdtemp(prefix='rlgs_live_%d_' % seed)
-    trace = os.path.join(work, 't.csv')
-    synth.write(df, trace)
-    ref = ref_runner.run_reference(trace, workdir=work, **flags)
-    tr = cpu_sim.prepare_trace(trace)
-    res = cpu_sim.run_fifo_yarn(cpu_sim.make_cluster(**flags), tr)
-    return seed, ref, cpu_sim.format_job_csv(tr, res), cpu_sim.format_cluster_csv(res)
+def _trace(df, rec):
+    """The trace as the reference read it: the CSV text, checked against the sha256 recorded with the reference's files."""
+    txt = df.to_csv(index=False)
+    assert goldutil.sha(txt) == rec['trace_sha256'], 'the random case generator drifted from the recording'
+    return cpu_sim.prepare_trace(pd.read_csv(io.StringIO(txt)))
 
 
-def test_oracle_equals_live_reference_on_random_cases():
-    with ThreadPoolExecutor(max_workers=6) as ex:
-        for seed, ref, job, clu in ex.map(_run, range(100, 112)):
-            assert ref['job_csv'] is not None, (seed, ref['stderr'][-500:])
-            assert job == ref['job_csv'], seed
-            assert clu == ref_runner.strip_util_column(ref['cluster_csv']), seed
+def test_oracle_equals_live_reference_on_random_cases(recorded):
+    for seed in golden_cases.RANDOM_FIFO:
+        ref = recorded[golden_cases.random_key('fifo', seed)]
+        df, flags = golden_cases.random_case(seed)
+        tr = _trace(df, ref)
+        res = cpu_sim.run_fifo_yarn(cpu_sim.make_cluster(**flags), tr)
+        assert ref['job_csv'] is not None, seed
+        assert cpu_sim.format_job_csv(tr, res) == ref['job_csv'], seed
+        assert cpu_sim.format_cluster_csv(res) == ref['cluster_csv'], seed
 
 
 # ---- the pack family: horus / horus+ / gandiva over the pack placement (zero utilisation spread: the reference's draws return
 # their mean) and over yarn (real spread); horus+ with its k-means draws injected (ref_runner._INJECT)
-PACK_COMBOS = [('horus', 'horus'), ('gandiva', 'gandiva'), ('horus+', 'horus+'), ('horus', 'yarn'), ('gandiva', 'yarn'), ('horus+', 'yarn')]
-
-
-def _run_pack(arg):
-    seed, (sched, scheme) = arg
-    df, flags = _case(seed)
-    if scheme != 'yarn':
-        df = df.copy(); df['gpu_utilization_max'] = df['gpu_utilization_avg']
-    rng = np.random.default_rng(seed + 7)
-    k = int(rng.integers(1, 8)); kq = int(rng.integers(1, 5)); inj = int(rng.integers(1, 1000))
-    work = tempfile.mkdtemp(prefix='rlgs_livepack_%d_' % seed)
-    trace = os.path.join(work, 't.csv')
-    synth.write(df, trace)
-    extra = dict(num_queue=kq, inject_seed=inj) if sched == 'horus+' else {}
-    ref = ref_runner.run_reference(trace, workdir=work, schedule=sched, scheme=scheme, num_buffer=k, **extra, **flags)
-    tr = cpu_sim.prepare_trace(trace)
-    try:
-        res = cpu_sim.run_pack(cpu_sim.make_cluster(**flags), tr, sched, k, scheme=('yarn' if scheme == 'yarn' else None),
-                               num_queue=kq, inject_seed=inj)
-    except RuntimeError:
-        return seed, sched, scheme, ref, None, None     # the oracle says the reference raises on this input
-    return seed, sched, scheme, ref, cpu_sim.format_job_csv(tr, res), cpu_sim.format_cluster_csv(res)
-
-
-def test_pack_oracle_equals_live_reference_on_random_cases():
-    args = [(200 + 3 * i + j, combo) for i, combo in enumerate(PACK_COMBOS) for j in range(2)]
-    with ThreadPoolExecutor(max_workers=6) as ex:
-        for seed, sched, scheme, ref, job, clu in ex.map(_run_pack, args):
-            if job is None:
-                assert ref['returncode'] != 0 or ref['job_csv'] is None or 'Error' in ref['stderr'], (seed, sched, scheme)
-                continue
-            assert ref['job_csv'] is not None, (seed, sched, scheme, ref['stderr'][-500:])
-            assert job == ref['job_csv'], (seed, sched, scheme)
-            assert clu == ref_runner.strip_util_column(ref['cluster_csv']), (seed, sched, scheme)
+def test_pack_oracle_equals_live_reference_on_random_cases(recorded):
+    for seed, (sched, scheme) in golden_cases.RANDOM_PACK:
+        ref = recorded[golden_cases.random_key('pack', seed, sched, scheme)]
+        df, flags, k, kq, inj = golden_cases.random_pack_case(seed, sched, scheme)
+        tr = _trace(df, ref)
+        try:
+            res = cpu_sim.run_pack(cpu_sim.make_cluster(**flags), tr, sched, k, scheme=('yarn' if scheme == 'yarn' else None),
+                                   num_queue=kq, inject_seed=inj)
+        except RuntimeError:   # the oracle says the reference raises on this input
+            assert ref['returncode'] != 0 or ref['job_csv'] is None or ref['stderr_has_error'], (seed, sched, scheme)
+            continue
+        assert ref['job_csv'] is not None, (seed, sched, scheme)
+        assert cpu_sim.format_job_csv(tr, res) == ref['job_csv'], (seed, sched, scheme)
+        assert cpu_sim.format_cluster_csv(res) == ref['cluster_csv'], (seed, sched, scheme)
 
 
 # ---- the legacy event loops: the reference's dead code run unmodified under the shim globals (oracle/ref_legacy_runner.py)
-LEGACY = ['sjf', 'shortest', 'shortest-gpu', 'dlas-gpu', 'dlas']
-
-
-def _run_legacy(arg):
-    import ref_legacy_runner
-    seed, sched = arg
-    df, flags = _case(seed)
-    rng = np.random.default_rng(seed + 11)
-    ql = tuple(int(x) for x in np.cumsum(rng.integers(5, 60, int(rng.integers(1, 4)))))   # 2 .. 4 queues
-    work = tempfile.mkdtemp(prefix='rlgs_liveleg_%d_' % seed)
-    trace = os.path.join(work, 't.csv')
-    synth.write(df, trace)
-    ref = ref_legacy_runner.run_legacy(trace, sched, workdir=work, queue_limit=ql, **flags)
-    tr = cpu_sim.prepare_trace(trace)
-    cluster = cpu_sim.make_cluster(**flags)
-    res, count = cpu_sim.run_legacy(cluster, tr, sched, ql)
-    return seed, sched, ref, cpu_sim.format_legacy_job_csv(tr, res, count), cpu_sim.format_legacy_cluster_csv(res, cluster, count)
-
-
-def test_legacy_oracle_equals_live_reference_on_random_cases():
-    args = [(300 + 5 * i + j, sched) for i, sched in enumerate(LEGACY) for j in range(2)]
-    with ThreadPoolExecutor(max_workers=6) as ex:
-        for seed, sched, ref, job, clu in ex.map(_run_legacy, args):
-            assert ref['job_csv'] is not None and ref['cluster_csv'] is not None, (seed, sched, ref['stderr'][-500:])
-            assert job == ref['job_csv'], (seed, sched)
-            assert clu == ref['cluster_csv'], (seed, sched)
+def test_legacy_oracle_equals_live_reference_on_random_cases(recorded):
+    for seed, sched in golden_cases.RANDOM_LEGACY:
+        ref = recorded[golden_cases.random_key('legacy', seed, sched)]
+        df, flags = golden_cases.random_case(seed)
+        tr = _trace(df, ref)
+        ql = golden_cases.random_legacy_queue_limit(seed)
+        cluster = cpu_sim.make_cluster(**flags)
+        res, count = cpu_sim.run_legacy(cluster, tr, sched, ql)
+        assert ref['job_csv'] is not None and ref['cluster_csv'] is not None, (seed, sched)
+        assert cpu_sim.format_legacy_job_csv(tr, res, count) == ref['job_csv'], (seed, sched)
+        assert cpu_sim.format_legacy_cluster_csv(res, cluster, count) == ref['cluster_csv'], (seed, sched)
